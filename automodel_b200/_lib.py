@@ -29,8 +29,8 @@ SIGNATURES = {
     "b200_embed_fwd": (_i, [_vp, _vp, _vp, _i, _i, _vp]),
     "b200_embed_bwd": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "b200_attn_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i64, _i64, _i64, _i64, _i, _i, _i, _i, _f, _vp]),
-    "b200_attn_bwd_workspace_bytes": (_sz, [_i, _i, _i]),
-    "b200_attn_bwd": (_i, [_vp] * 11 + [_i, _i] + [_i64] * 8 + [_i, _i, _i, _i, _f, _vp]),
+    "b200_attn_bwd_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "b200_attn_bwd": (_i, [_vp] * 10 + [_sz, _vp] + [_i, _i] + [_i64] * 8 + [_i, _i, _i, _i, _f, _vp]),
     "b200_ce_fwd_bwd": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i64, _i64, _i, _vp]),
     "b200_sumsq_workspace_floats": (_i, []),
     "b200_sumsq_bf16": (_i, [_vp, _i64, _vp, _vp, _i, _vp]),

@@ -442,13 +442,17 @@ __global__ void __launch_bounds__(128) attn_bwd_kernel(const __nv_bfloat16* __re
 
 // dq (bf16, strided) = scale * dq_acc (fp32)
 __global__ void __launch_bounds__(256) attn_dq_convert_kernel(const float* __restrict__ acc, __nv_bfloat16* __restrict__ dq, int64_t T,
-                                                             int cols, int64_t ld_acc, int64_t lddq, float scale) {
+                                                             int cols, int64_t ld_acc, int64_t lddq, float scale, int nbuf) {
   const int vpr = cols / 4;
   const int64_t total = T * vpr;
   for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < total; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int64_t t = i / vpr;
     const int c = static_cast<int>(i - t * vpr);
-    const float4 a = *reinterpret_cast<const float4*>(acc + t * ld_acc + c * 4);
+    float4 a = *reinterpret_cast<const float4*>(acc + t * ld_acc + c * 4);
+    for (int b = 1; b < nbuf; ++b) {  // further accumulators (one per CTA, T rows each), summed in a fixed order
+      const float4 x = *reinterpret_cast<const float4*>(acc + (b * T + t) * ld_acc + c * 4);
+      a.x += x.x; a.y += x.y; a.z += x.z; a.w += x.w;
+    }
     uint2 o;
     o.x = pack_bf16x2(a.x * scale, a.y * scale);
     o.y = pack_bf16x2(a.z * scale, a.w * scale);
@@ -464,11 +468,11 @@ int attn_delta_launch(const void* o, const void* dout, float* delta, int64_t ldo
   B200_CHECK_LAUNCH("attn_delta");
   return 0;
 }
-int attn_dq_convert_launch(const float* acc, void* dq, int64_t T, int cols, int64_t lddq, float scale, cudaStream_t st) {
+int attn_dq_convert_launch(const float* acc, int nbuf, void* dq, int64_t T, int cols, int64_t lddq, float scale, cudaStream_t st) {
   const int64_t total = T * (cols / 4);
   int blocks = static_cast<int>((total + 255) / 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
-  attn_dq_convert_kernel<<<blocks, 256, 0, st>>>(acc, static_cast<__nv_bfloat16*>(dq), T, cols, cols, lddq, scale);
+  attn_dq_convert_kernel<<<blocks, 256, 0, st>>>(acc, static_cast<__nv_bfloat16*>(dq), T, cols, cols, lddq, scale, nbuf);
   B200_CHECK_LAUNCH("attn_dq_convert");
   return 0;
 }
@@ -501,8 +505,10 @@ int attn_fwd(const void* q, const void* k, const void* v, void* o, float* lse, c
   return set_error(B200_ERR_UNSUPPORTED, "attn: head_dim %d not in {64,128}", D);
 }
 
-size_t attn_bwd_workspace_bytes(int T, int Hq, int D) {
-  return static_cast<size_t>(T) * Hq * D * sizeof(float) + static_cast<size_t>(T) * Hq * sizeof(float);
+size_t attn_bwd_workspace_bytes(int T, int Hq, int D, int max_seqlen) {
+  // fp32 dQ accumulator + delta; a second accumulator when no sequence is longer than 512 tokens (attn_bwd_tc: bit-reproducible dQ)
+  const size_t acc = static_cast<size_t>(T) * Hq * D * sizeof(float);
+  return (max_seqlen <= 512 ? 2 : 1) * acc + static_cast<size_t>(T) * Hq * sizeof(float);
 }
 
 template <int D>
@@ -534,16 +540,17 @@ static int attn_bwd_launch(const void* q, const void* k, const void* v, const vo
     const int64_t total = static_cast<int64_t>(T) * (cols / 4);
     int blocks = static_cast<int>((total + 255) / 256);
     if (blocks > 148 * 8) blocks = 148 * 8;
-    attn_dq_convert_kernel<<<blocks, 256, 0, st>>>(dq_acc, static_cast<__nv_bfloat16*>(dq), T, cols, cols, lddq, scale);
+    attn_dq_convert_kernel<<<blocks, 256, 0, st>>>(dq_acc, static_cast<__nv_bfloat16*>(dq), T, cols, cols, lddq, scale, 1);
     B200_CHECK_LAUNCH("attn_dq_convert");
   }
   return 0;
 }
 
 int attn_bwd(const void* q, const void* k, const void* v, const void* o, const void* dout, const float* lse, void* dq, void* dk,
-             void* dv, void* ws, const int* cu_seqlens, int nseq, int max_len, int64_t ldq, int64_t ldk, int64_t ldv, int64_t ldo,
-             int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv, int D, int T, float scale, cudaStream_t st) {
+             void* dv, void* ws, size_t ws_bytes, const int* cu_seqlens, int nseq, int max_len, int64_t ldq, int64_t ldk, int64_t ldv,
+             int64_t ldo, int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv, int D, int T, float scale, cudaStream_t st) {
   if (Hq % Hkv) return set_error(B200_ERR_ARG, "attn: Hq %% Hkv != 0");
+  if (ws_bytes < static_cast<size_t>(T) * Hq * (D + 1) * sizeof(float)) return set_error(B200_ERR_ARG, "attn_bwd: workspace of %zu bytes is too small", ws_bytes);
   if ((ldq | ldk | ldv | ldo | lddo | lddq | lddk | lddv) % 8) return set_error(B200_ERR_ARG, "attn: row pitches must be multiples of 8 elements");
   if (D == 128)
     return attn_bwd_launch<128>(q, k, v, o, dout, lse, dq, dk, dv, ws, cu_seqlens, nseq, max_len, ldq, ldk, ldv, ldo, lddo, lddq, lddk,

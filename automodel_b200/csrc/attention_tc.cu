@@ -374,7 +374,7 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
                    const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmDO,
                    const __grid_constant__ CUtensorMap tmDQ, const float* __restrict__ lse, const float* __restrict__ delta,
                    __nv_bfloat16* __restrict__ dk, __nv_bfloat16* __restrict__ dv, const int* __restrict__ cu_seqlens,
-                   int64_t lddk, int64_t lddv, int Hq, int Hkv, int T, float scale, float scale_log2) {
+                   int64_t lddk, int64_t lddv, int Hq, int Hkv, int T, float scale, float scale_log2, int dq_cta_rows) {
   using L = AttnBwdSmem<D>;
   constexpr int ATOMS = D / 64;
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -695,7 +695,8 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {  // one [32 rows x 32 floats] box per warp: no cross-warp barrier, 16 reductions in flight per CTA
-          tma_reduce_add_2d(&tmDQ, smem + L::PT_OFF + chunk * 16384 + quad * 4096, h * D + chunk * 32, s0 + m0 + quad * 32);
+          tma_reduce_add_2d(&tmDQ, smem + L::PT_OFF + chunk * 16384 + quad * 4096, h * D + chunk * 32,
+                            static_cast<int>(blockIdx.x) * dq_cta_rows + s0 + m0 + quad * 32);
           tma_store_commit();
         }
       }
@@ -744,13 +745,13 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 }
 
 int attn_delta_launch(const void* o, const void* dout, float* delta, int64_t ldo, int64_t lddo, int Hq, int D, int T, cudaStream_t st);
-int attn_dq_convert_launch(const float* acc, void* dq, int64_t T, int cols, int64_t lddq, float scale, cudaStream_t st);
+int attn_dq_convert_launch(const float* acc, int nbuf, void* dq, int64_t T, int cols, int64_t lddq, float scale, cudaStream_t st);
 
 template <int D>
 static int attn_bwd_tc_launch(const void* q, const void* k, const void* v, const void* o, const void* dout, const float* lse, void* dq,
-                              void* dk, void* dv, void* ws, const int* cu, int nseq, int max_len, int64_t ldq, int64_t ldk, int64_t ldv,
-                              int64_t ldo, int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv, int T, float scale,
-                              cudaStream_t st) {
+                              void* dk, void* dv, void* ws, size_t ws_bytes, const int* cu, int nseq, int max_len, int64_t ldq, int64_t ldk,
+                              int64_t ldv, int64_t ldo, int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv, int T,
+                              float scale, cudaStream_t st) {
   using L = AttnBwdSmem<D>;
   auto kern = attn_bwd_tc_kernel<D>;
   static bool configured = false;
@@ -759,21 +760,31 @@ static int attn_bwd_tc_launch(const void* q, const void* k, const void* v, const
     if (e != cudaSuccess) return set_error(B200_ERR_CUDA, "attn_bwd_tc smem attr: %s", cudaGetErrorString(e));
     configured = true;
   }
+  // The dQ tiles of one (sequence, kv head) come from `pairs` CTAs, and each CTA adds at most two tiles to an element (one per kv tile
+  // it owns), so with one fp32 accumulator per CTA every element is summed in a fixed order and dQ is bit-reproducible.  That costs
+  // `pairs` accumulators of memset and read-back, so it is done for two CTAs (longest sequence 257..512 tokens) when the caller sized
+  // the workspace for it (attn_bwd_workspace_bytes with max_seqlen <= 512); otherwise the CTAs share one accumulator and the order of
+  // the fp32 additions follows their timing (last-bit differences from launch to launch).  One CTA adds at most two tiles anyway.
+  const int pairs = ((max_len + 127) / 128 + 1) / 2;
+  const size_t acc_elems = static_cast<size_t>(T) * Hq * D;
+  const size_t delta_bytes = static_cast<size_t>(T) * Hq * sizeof(float);
+  if (ws_bytes < acc_elems * sizeof(float) + delta_bytes) return set_error(B200_ERR_ARG, "attn_bwd: workspace of %zu bytes is too small", ws_bytes);
+  const int nbuf = pairs == 2 && ws_bytes >= 2 * acc_elems * sizeof(float) + delta_bytes ? 2 : 1;
   float* dq_acc = static_cast<float*>(ws);
-  float* delta = dq_acc + static_cast<size_t>(T) * Hq * D;
-  cudaError_t e = cudaMemsetAsync(dq_acc, 0, static_cast<size_t>(T) * Hq * D * sizeof(float), st);
+  float* delta = dq_acc + nbuf * acc_elems;
+  cudaError_t e = cudaMemsetAsync(dq_acc, 0, nbuf * acc_elems * sizeof(float), st);
   if (e != cudaSuccess) return set_error(B200_ERR_CUDA, "attn_bwd memset: %s", cudaGetErrorString(e));
   int rc;
   if ((rc = attn_delta_launch(o, dout, delta, ldo, lddo, Hq, D, T, st))) return rc;
   CUtensorMap tq, tk, tv, tdo, tdq;
-  if ((rc = make_tmap_2d_f32(&tdq, dq_acc, T, static_cast<uint64_t>(Hq) * D, static_cast<uint64_t>(Hq) * D, 32, 32))) return rc;
+  if ((rc = make_tmap_2d_f32(&tdq, dq_acc, static_cast<uint64_t>(nbuf) * T, static_cast<uint64_t>(Hq) * D, static_cast<uint64_t>(Hq) * D, 32, 32))) return rc;
   if ((rc = make_tmap_2d_bf16(&tq, q, T, static_cast<uint64_t>(Hq) * D, ldq, 64, 128))) return rc;
   if ((rc = make_tmap_2d_bf16(&tk, k, T, static_cast<uint64_t>(Hkv) * D, ldk, 64, 128))) return rc;
   if ((rc = make_tmap_2d_bf16(&tv, v, T, static_cast<uint64_t>(Hkv) * D, ldv, 64, 128))) return rc;
   if ((rc = make_tmap_2d_bf16(&tdo, dout, T, static_cast<uint64_t>(Hq) * D, lddo, 64, 128))) return rc;
   dim3 grid(((max_len + 127) / 128 + 1) / 2, Hkv, nseq);
   kern<<<grid, 576, L::DYN, st>>>(tq, tk, tv, tdo, tdq, lse, delta, static_cast<__nv_bfloat16*>(dk), static_cast<__nv_bfloat16*>(dv), cu,
-                                  lddk, lddv, Hq, Hkv, T, scale, scale * 1.4426950408889634f);
+                                  lddk, lddv, Hq, Hkv, T, scale, scale * 1.4426950408889634f, nbuf > 1 ? T : 0);
   B200_CHECK_LAUNCH("attn_bwd_tc");
 #ifdef B200_ATTN_PROFILE
   {
@@ -788,19 +799,19 @@ static int attn_bwd_tc_launch(const void* q, const void* k, const void* v, const
     cudaMemcpyToSymbol(g_attn_prof, z, sizeof(z));
   }
 #endif
-  return attn_dq_convert_launch(dq_acc, dq, T, Hq * D, lddq, scale, st);
+  return attn_dq_convert_launch(dq_acc, nbuf, dq, T, Hq * D, lddq, scale, st);
 }
 
 int attn_bwd_tc(const void* q, const void* k, const void* v, const void* o, const void* dout, const float* lse, void* dq, void* dk,
-                void* dv, void* ws, const int* cu_seqlens, int nseq, int max_len, int64_t ldq, int64_t ldk, int64_t ldv, int64_t ldo,
-                int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv, int D, int T, float scale, cudaStream_t st) {
+                void* dv, void* ws, size_t ws_bytes, const int* cu_seqlens, int nseq, int max_len, int64_t ldq, int64_t ldk, int64_t ldv,
+                int64_t ldo, int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv, int D, int T, float scale, cudaStream_t st) {
   if (Hq % Hkv) return set_error(B200_ERR_ARG, "attn: Hq %% Hkv != 0");
   if ((ldq | ldk | ldv | ldo | lddo | lddq | lddk | lddv) % 8) return set_error(B200_ERR_ARG, "attn: row pitches must be multiples of 8 elements");
   if (D == 128)
-    return attn_bwd_tc_launch<128>(q, k, v, o, dout, lse, dq, dk, dv, ws, cu_seqlens, nseq, max_len, ldq, ldk, ldv, ldo, lddo, lddq, lddk,
+    return attn_bwd_tc_launch<128>(q, k, v, o, dout, lse, dq, dk, dv, ws, ws_bytes, cu_seqlens, nseq, max_len, ldq, ldk, ldv, ldo, lddo, lddq, lddk,
                                    lddv, Hq, Hkv, T, scale, st);
   if (D == 64)
-    return attn_bwd_tc_launch<64>(q, k, v, o, dout, lse, dq, dk, dv, ws, cu_seqlens, nseq, max_len, ldq, ldk, ldv, ldo, lddo, lddq, lddk,
+    return attn_bwd_tc_launch<64>(q, k, v, o, dout, lse, dq, dk, dv, ws, ws_bytes, cu_seqlens, nseq, max_len, ldq, ldk, ldv, ldo, lddo, lddq, lddk,
                                   lddv, Hq, Hkv, T, scale, st);
   return set_error(B200_ERR_UNSUPPORTED, "attn: head_dim %d not in {64,128}", D);
 }

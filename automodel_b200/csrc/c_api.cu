@@ -41,13 +41,13 @@ int adamw_step(void*, const void*, void*, void*, float*, int64_t, float, float, 
 int add_inplace_bf16(void*, const void*, int64_t, cudaStream_t);
 int attn_fwd(const void*, const void*, const void*, void*, float*, const int*, int, int, int64_t, int64_t, int64_t, int64_t, int, int,
              int, int, float, cudaStream_t);
-size_t attn_bwd_workspace_bytes(int, int, int);
-int attn_bwd(const void*, const void*, const void*, const void*, const void*, const float*, void*, void*, void*, void*, const int*, int,
+size_t attn_bwd_workspace_bytes(int, int, int, int);
+int attn_bwd(const void*, const void*, const void*, const void*, const void*, const float*, void*, void*, void*, void*, size_t, const int*, int,
              int, int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, int, int, int, int, float, cudaStream_t);
 
 int attn_fwd_tc(const void*, const void*, const void*, void*, float*, const int*, int, int, int64_t, int64_t, int64_t, int64_t, int, int,
                 int, int, float, cudaStream_t);
-int attn_bwd_tc(const void*, const void*, const void*, const void*, const void*, const float*, void*, void*, void*, void*, const int*, int,
+int attn_bwd_tc(const void*, const void*, const void*, const void*, const void*, const float*, void*, void*, void*, void*, size_t, const int*, int,
                 int, int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, int64_t, int, int, int, int, float, cudaStream_t);
 
 struct CommCtx;
@@ -135,7 +135,7 @@ static inline cudaStream_t S(b200_stream_t s) { return reinterpret_cast<cudaStre
 extern "C" {
 
 const char* b200_last_error(void) { return g_err; }
-int b200_abi_version(void) { return 1; }
+int b200_abi_version(void) { return 2; }
 int b200_set_option(const char* name, int value) {
   if (name && !strcmp(name, "attn_impl")) { g_attn_impl = value; return 0; }
   if (name && !strcmp(name, "attn_fwd_variant")) { g_attn_fwd_variant = value; return 0; }
@@ -206,15 +206,17 @@ int b200_attn_fwd(const void* q, const void* k, const void* v, void* o, float* l
     return attn_fwd_tc(q, k, v, o, lse, cu_seqlens, nseq, max_seqlen, ldq, ldk, ldv, ldo, Hq, Hkv, head_dim, total_tokens, scale, S(stream));
   return attn_fwd(q, k, v, o, lse, cu_seqlens, nseq, max_seqlen, ldq, ldk, ldv, ldo, Hq, Hkv, head_dim, total_tokens, scale, S(stream));
 }
-size_t b200_attn_bwd_workspace_bytes(int total_tokens, int Hq, int head_dim) { return attn_bwd_workspace_bytes(total_tokens, Hq, head_dim); }
+size_t b200_attn_bwd_workspace_bytes(int total_tokens, int Hq, int head_dim, int max_seqlen) {
+  return attn_bwd_workspace_bytes(total_tokens, Hq, head_dim, max_seqlen);
+}
 int b200_attn_bwd(const void* q, const void* k, const void* v, const void* o, const void* dout, const float* lse, void* dq, void* dk,
-                  void* dv, void* workspace, const int* cu_seqlens, int nseq, int max_seqlen, int64_t ldq, int64_t ldk, int64_t ldv,
-                  int64_t ldo, int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv, int head_dim, int total_tokens,
-                  float scale, b200_stream_t stream) {
+                  void* dv, void* workspace, size_t workspace_bytes, const int* cu_seqlens, int nseq, int max_seqlen, int64_t ldq,
+                  int64_t ldk, int64_t ldv, int64_t ldo, int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq, int Hkv,
+                  int head_dim, int total_tokens, float scale, b200_stream_t stream) {
   if (g_attn_impl == 1)
-    return attn_bwd_tc(q, k, v, o, dout, lse, dq, dk, dv, workspace, cu_seqlens, nseq, max_seqlen, ldq, ldk, ldv, ldo, lddo, lddq, lddk,
+    return attn_bwd_tc(q, k, v, o, dout, lse, dq, dk, dv, workspace, workspace_bytes, cu_seqlens, nseq, max_seqlen, ldq, ldk, ldv, ldo, lddo, lddq, lddk,
                        lddv, Hq, Hkv, head_dim, total_tokens, scale, S(stream));
-  return attn_bwd(q, k, v, o, dout, lse, dq, dk, dv, workspace, cu_seqlens, nseq, max_seqlen, ldq, ldk, ldv, ldo, lddo, lddq, lddk, lddv,
+  return attn_bwd(q, k, v, o, dout, lse, dq, dk, dv, workspace, workspace_bytes, cu_seqlens, nseq, max_seqlen, ldq, ldk, ldv, ldo, lddo, lddq, lddk, lddv,
                   Hq, Hkv, head_dim, total_tokens, scale, S(stream));
 }
 int b200_ce_fwd_bwd(void* logits, const int* labels, float* row_loss, float* loss_out, int rows, int vocab, int64_t ld,

@@ -274,7 +274,8 @@ class ShardedLlamaEngine:
         if self.device.type == "cuda":
             from ._lib import lib
             self.norm_ws = torch.empty(lib().b200_rmsnorm_bwd_workspace_floats(T, h), dtype=torch.float32, device=dev)
-            self.attn_ws = torch.empty(lib().b200_attn_bwd_workspace_bytes(T, d.heads, d.head_dim), dtype=torch.uint8, device=dev)
+            # sized for the longest sequence this engine can see (the RoPE tables bound it)
+            self.attn_ws = torch.empty(lib().b200_attn_bwd_workspace_bytes(T, d.heads, d.head_dim, min(T, n_pos)), dtype=torch.uint8, device=dev)
         else:
             self.norm_ws = self.attn_ws = None
         self.loss_dev = torch.zeros(1, dtype=torch.float32, device=dev)
@@ -413,15 +414,19 @@ class ShardedLlamaEngine:
                 self._rs_started = True
 
         if st.cuda:
+            # N = 1 has no collective: the copy and the grad-norm partial go to the stream where _reduce_scatter_unit takes the resident
+            # units' partials.  Every partial then adds into norm_sq in issue order (the resident engine's order), and no two sumsq_ calls
+            # share the device's sumsq workspace from different streams at once.
+            side = st.opt if self.world == 1 and self.replicas == 1 else st.comm
             ev = st.event()
             st.record(ev)
             wg = self._wg_last if self._wg_on else None
-            with torch.cuda.stream(st.comm):
-                st.wait(ev, st.comm)
-                st.wait(wg, st.comm)
+            with torch.cuda.stream(side):
+                st.wait(ev, side)
+                st.wait(wg, side)
                 body()
                 done = st.event()
-                st.record(done, st.comm)
+                st.record(done, side)
                 self.ev_rs[ui] = done
                 self._gslot_rs[k] = done
         else:

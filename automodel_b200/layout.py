@@ -168,7 +168,8 @@ def memory_plan(d: LlamaDims, world: int, tokens: int, reshard_after_forward: bo
     optim = (2 + 2 + (4 if master_weights else 0)) * (P // world)
     per_layer = 2 * T * (h * 5 + d.qkv_cols + d.q_cols + 3 * F) + 4 * T * (2 + d.heads)      # x1, h1, x2, (h counted below) qkv, o2, gu (2F), a (F); rstd x2, lse
     acts = 2 * T * h * (L + 1) + (per_layer if activation_checkpointing else per_layer * L)
-    tmp = 2 * T * (4 * h + 3 * F + d.q_cols + d.qkv_cols) + 2 * T * d.vocab + 4 * T * h    # backward scratch, logits, attention dq accumulator (fp32, Hq*D = h)
+    dq_accs = 2 if min(T, d.max_pos) <= 512 else 1        # attention dQ accumulators (fp32, Hq*D = h): two for sequences of <= 512 tokens
+    tmp = 2 * T * (4 * h + 3 * F + d.q_cols + d.qkv_cols) + 2 * T * d.vocab + 4 * T * h * dq_accs     # backward scratch, logits, dQ
     staging = 4 * (max(padded) + max(padded) // world) if world > 1 else 0                   # fp32 reduce staging of the NCCL path
     total = params + grads + optim + acts + tmp + staging
     return {"params": params, "grads": grads, "optimizer": optim, "activations": acts, "scratch_logits": tmp, "fp32_reduce_staging": staging, "total": total}

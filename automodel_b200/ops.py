@@ -254,11 +254,10 @@ def attn_fwd(q, k, v, cu_seqlens, max_seqlen, Hq, Hkv, D, scale=None, out=None, 
 def attn_bwd(q, k, v, o, dout, lse, cu_seqlens, max_seqlen, Hq, Hkv, D, dq, dk, dv, scale=None, workspace=None):
     T = q.shape[0]
     scale = scale if scale is not None else D ** -0.5
-    need = lib().b200_attn_bwd_workspace_bytes(T, Hq, D)
-    if workspace is None or workspace.numel() < need:
-        workspace = torch.empty(need, dtype=torch.uint8, device=q.device)
+    if workspace is None:
+        workspace = torch.empty(lib().b200_attn_bwd_workspace_bytes(T, Hq, D, max_seqlen), dtype=torch.uint8, device=q.device)
     check(lib().b200_attn_bwd(q.data_ptr(), k.data_ptr(), v.data_ptr(), o.data_ptr(), dout.data_ptr(), lse.data_ptr(), dq.data_ptr(),
-                              dk.data_ptr(), dv.data_ptr(), workspace.data_ptr(), cu_seqlens.data_ptr(), cu_seqlens.numel() - 1,
+                              dk.data_ptr(), dv.data_ptr(), workspace.data_ptr(), workspace.numel(), cu_seqlens.data_ptr(), cu_seqlens.numel() - 1,
                               max_seqlen, q.stride(0), k.stride(0), v.stride(0), o.stride(0), dout.stride(0), dq.stride(0),
                               dk.stride(0), dv.stride(0), Hq, Hkv, D, T, float(scale), _st()), "b200_attn_bwd")
     _count(3)

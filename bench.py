@@ -5,6 +5,8 @@
   python bench.py --impl reference --gpus N ...            reference arm: the UNMODIFIED reference recipe (baseline/_ref install) on
                                                            the host cores, CPU/gloo, bounded sample (falls back to the numpy
                                                            restatement in oracle/ when the install is absent)
+  python bench.py --steps K --dump-outputs DIR             also write what the last timed step computed to DIR/<name>.npy, to
+                                                           compare two builds output for output (inputs and init are seeded)
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for what each field means.
 """
@@ -43,6 +45,29 @@ def measured_peaks():
         d = json.load(open(p))
         return {"hbm_gbs": d["hbm_gbs"], "tflops_burst": d["bf16_tflops"], "tflops_sustained": d["bf16_tflops_sustained"], "source": "measured"}
     return {"hbm_gbs": 6650.0, "tflops_burst": 1590.0, "tflops_sustained": 1400.0, "source": "fallback"}
+
+
+DUMP_SAMPLE = 16384     # elements kept per parameter tensor: the 291 tensors of Llama-3-8B come to 16 MB of float32
+
+
+def dump_outputs(out_dir, loss, grad_norm, params):
+    """What one training step hands its caller, as float32 .npy files in out_dir: loss.npy, grad_norm.npy and one file per updated
+    parameter (HF name).  A parameter of more than DUMP_SAMPLE elements is sampled at fixed, distinct indices seeded by its name, so that two
+    builds run with the same arguments can be compared file by file.  Compare with a tolerance: the attention backward adds dQ tiles
+    in whatever order its CTAs finish, and at these shapes dQ differs in its last bits from launch to launch (50 of 50 launches on a
+    B200 at 1000 W), so two runs of one build agree to rounding, not bit for bit."""
+    import zlib
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([float(loss)], dtype=np.float32))
+    np.save(os.path.join(out_dir, "grad_norm.npy"), np.array([float(grad_norm)], dtype=np.float32))
+    for name, p in params.items():
+        flat = p.reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(zlib.crc32(name.encode())).choice(flat.numel(), DUMP_SAMPLE, replace=False))
+            flat = flat.index_select(0, torch.from_numpy(idx).to(flat.device))
+        np.save(os.path.join(out_dir, name + ".npy"), flat.float().cpu().numpy())
 
 
 class ClockSampler:
@@ -185,7 +210,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="N > 1 only: skip the correctness block that precedes the timed region")
     ap.add_argument("--profile", action="store_true", help="for ncu runs only: 1 warm-up step, no e2e leg, no CPU baseline (numbers printed are NOT bench values)")
     ap.add_argument("--adam-mode", type=int, default=1, help="1 = torch.optim.AdamW bf16 op sequence (reference default optimizer), 0 = fp32 math")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's loss, grad norm and (sampled) updated parameters to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -291,6 +322,8 @@ def main():
     if args.profile:
         torch.cuda.profiler.stop()
     launches = ops.LAUNCHES - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, gn, eng.state_dict())
     # pure host cost of enqueueing one step: start from an idle GPU so the launch queue never back-pressures
     torch.cuda.synchronize()
     h0 = time.perf_counter()
@@ -364,8 +397,9 @@ def main():
     eng.h2d_bytes = 0
     w0 = time.perf_counter()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e2e_steps = 1 if args.profile else args.steps
     e0.record()
-    for i in range(1 if args.profile else args.steps):
+    for i in range(e2e_steps):
         l, g_ = e2e_step(host[i % nbatch])
         lv, gv = float(l), float(g_)         # D2H read of the step result (host sync, as the reference recipe does every step)
     eng.sync_params()
@@ -374,8 +408,8 @@ def main():
     e2e_ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(e2e_ms, op=dist.ReduceOp.MAX)
-    e2e_ms_step = float(e2e_ms.item()) / args.steps
-    h2d = eng.h2d_bytes // args.steps
+    e2e_ms_step = float(e2e_ms.item()) / e2e_steps
+    h2d = eng.h2d_bytes // e2e_steps
     e2e = {"value": tokens_per_step / (e2e_ms_step / 1e3), "unit": "tokens/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": 8,
            "ms_per_step": e2e_ms_step, "host_threads": 1, "api": "ShardedLlamaEngine.train_step" if args.e2e_api == "engine" else "B200CausalLM facade (recipe call sequence)"}
 

@@ -94,9 +94,12 @@ int b200_embed_bwd(const int* ids, const void* dh, void* dW, int* workspace, int
 int b200_attn_fwd(const void* q, const void* k, const void* v, void* o, float* lse, const int* cu_seqlens, int nseq,
                   int max_seqlen, int64_t ldq, int64_t ldk, int64_t ldv, int64_t ldo, int Hq, int Hkv, int head_dim,
                   int total_tokens, float scale, b200_stream_t stream);
-size_t b200_attn_bwd_workspace_bytes(int total_tokens, int Hq, int head_dim);
+/* Workspace for batches of `total_tokens` tokens whose sequences are at most `max_seqlen` long.  With max_seqlen <= 512 it includes a
+ * second fp32 dQ accumulator, and dQ of sequences of 257..512 tokens is then bit-reproducible; otherwise dQ may differ from launch to
+ * launch in its last bits (fp32 additions in the order the CTAs finish).  b200_attn_bwd takes the size it was given. */
+size_t b200_attn_bwd_workspace_bytes(int total_tokens, int Hq, int head_dim, int max_seqlen);
 int b200_attn_bwd(const void* q, const void* k, const void* v, const void* o, const void* dout, const float* lse, void* dq,
-                  void* dk, void* dv, void* workspace, const int* cu_seqlens, int nseq, int max_seqlen, int64_t ldq,
+                  void* dk, void* dv, void* workspace, size_t workspace_bytes, const int* cu_seqlens, int nseq, int max_seqlen, int64_t ldq,
                   int64_t ldk, int64_t ldv, int64_t ldo, int64_t lddo, int64_t lddq, int64_t lddk, int64_t lddv, int Hq,
                   int Hkv, int head_dim, int total_tokens, float scale, b200_stream_t stream);
 

@@ -25,7 +25,7 @@ def test_header_symbols_exported_and_bound():
         assert hasattr(h, n), f"{n} declared in include/b200_train.h but not exported"
         assert n in SIGNATURES, f"{n} has no ctypes signature in automodel_b200/_lib.py"
     assert set(SIGNATURES) <= set(names), set(SIGNATURES) - set(names)
-    assert lib().b200_abi_version() == 1
+    assert lib().b200_abi_version() == 2
 
 
 def test_errors_are_reported_not_raised():
@@ -67,7 +67,7 @@ def test_header_is_plain_c_and_binds_from_a_c_program(tmp_path):
 #include <string.h>
 #include "b200_train.h"
 int main(void) {
-  if (b200_abi_version() != 1) return 1;
+  if (b200_abi_version() != 2) return 1;
   if (b200_set_option("gemm_sched", 0) != 0) return 2;
   if (b200_set_option("no_such_option", 1) >= 0) return 3;
   if (strlen(b200_last_error()) == 0) return 4;
@@ -82,4 +82,4 @@ int main(void) {
     subprocess.run([gcc, "-std=c99", "-Wall", "-I", inc, str(src), "-o", str(exe), "-L", libdir, "-lb200_train", f"-Wl,-rpath,{libdir}"], check=True)
     r = subprocess.run([str(exe)], capture_output=True, text=True)
     assert r.returncode == 0, (r.returncode, r.stdout, r.stderr)
-    assert "abi 1 ok" in r.stdout
+    assert "abi 2 ok" in r.stdout

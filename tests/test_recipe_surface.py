@@ -1,8 +1,10 @@
 """The reference-facing facade (automodel_b200/recipe.py) driven exactly the way the reference recipe drives its model
 (recipes/llm/train_ft.py:1357-1473, 1482-1635): model(**batch).logits -> loss_fn(logits, labels, num_label_tokens) ->
 (loss * dp).backward() -> clip -> optimizer.step().  Runs on CPU with the stand-in kernels; parity target = the reference fixtures.
-When /root/reference is importable the reference's own MaskedCrossEntropy is the loss function."""
-import sys
+The reference's MaskedCrossEntropy is the loss function, restated and pinned to the reference's own outputs
+(tests/golden/surface_golden.npz, written by tests/golden/gen_surface_golden.py)."""
+import os
+import numpy as np
 import pytest
 import torch
 
@@ -10,25 +12,24 @@ from automodel_b200.recipe import B200ShardedConfig, B200ShardedManager, B200Mas
 from tests import cpu_kernels
 from tests.golden_utils import load, model_cfg, init_params, batches
 
-
-def _reference_masked_ce():
-    try:
-        sys.path.insert(0, "/root/reference")
-        from nemo_automodel.components.loss.masked_ce import MaskedCrossEntropy  # noqa
-        return MaskedCrossEntropy()
-    except Exception:
-        return None
-    finally:
-        if sys.path[0] == "/root/reference":
-            sys.path.pop(0)
+SURFACE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "surface_golden.npz")
 
 
 class _TorchMaskedCE(torch.nn.Module):
-    """components/loss/masked_ce.py:73-89 restated (used when the reference is not importable, e.g. on the GPU box)."""
+    """components/loss/masked_ce.py:73-89 restated."""
 
     def forward(self, logits, labels, mask=None, num_label_tokens=None):
         loss = torch.nn.functional.cross_entropy(logits.view(-1, logits.size(-1)).float(), labels.view(-1), reduction="sum", ignore_index=-100)
         return loss / num_label_tokens
+
+
+@pytest.mark.parametrize("dtype", ["float32", "bfloat16"])
+def test_restated_masked_ce_equals_the_reference_golden(dtype):
+    """The restatement returns, bit for bit, what the reference's MaskedCrossEntropy returned on the same logits and labels."""
+    z = np.load(SURFACE)
+    logits = torch.from_numpy(z["ce/logits"]).to(getattr(torch, dtype))
+    loss = _TorchMaskedCE()(logits, torch.from_numpy(z["ce/labels"]), num_label_tokens=int(z["ce/num_label_tokens"]))
+    assert float(loss) == float(z[f"ce/loss_{dtype}"]), (float(loss), float(z[f"ce/loss_{dtype}"]))
 
 
 class _Cfg:
@@ -65,7 +66,7 @@ def _run_recipe_loop(loss_kind, device, ops):
     if loss_kind == "fused_loss":
         loss_fn = B200MaskedCrossEntropy()
     else:
-        loss_fn = _reference_masked_ce() or _TorchMaskedCE()
+        loss_fn = _TorchMaskedCE()
     dp = 1
     for s in range(len(meta["loss"])):
         mbs = batches(z, meta, s)
@@ -191,17 +192,10 @@ def test_foreign_optimizer_is_detected():
 
 def test_strategy_config_accepts_an_fsdp2_yaml_and_refuses_what_it_cannot_honour():
     """Every FSDP2Config key is a B200ShardedConfig key (so `_validate_strategy_kwargs`, recipes/_dist_setup.py:44-54, lets an FSDP2 YAML
-    through with only `strategy:` changed); keys that would change the computation raise."""
+    through with only `strategy:` changed); keys that would change the computation raise.  FSDP2Config's field names: golden data."""
     import dataclasses
-    try:
-        sys.path.insert(0, "/root/reference")
-        from nemo_automodel.components.distributed.config import FSDP2Config
-        theirs = {f.name for f in dataclasses.fields(FSDP2Config)}
-    except Exception:
-        theirs = {"sequence_parallel", "tp_plan", "mp_policy", "offload_policy", "activation_checkpointing", "defer_fsdp_grad_sync", "backend"}
-    finally:
-        if sys.path[0] == "/root/reference":
-            sys.path.pop(0)
+    theirs = set(np.load(SURFACE)["fsdp2_config_fields"].tolist())
+    assert len(theirs) == 14 and {"mp_policy", "tp_plan", "defer_fsdp_grad_sync"} <= theirs
     ours = {f.name for f in dataclasses.fields(B200ShardedConfig)}
     assert theirs <= ours, sorted(theirs - ours)
     B200ShardedConfig(defer_fsdp_grad_sync=False, enable_fsdp2_prefetch=True, fsdp2_backward_prefetch_depth=1, backend="gloo")
